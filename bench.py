@@ -26,6 +26,9 @@ per-rank tables exactly over NCCL.
              box's host cores, on a bounded sample of the same workload.  Reported, not the target.
 
 --impl reference times only that CPU path (rank 0; other ranks exit) and prints the same JSON shape.
+
+--dump-outputs DIR writes the tables the last timed step returned (rank 0) as float64 .npy files, so that two builds
+can be compared output for output: the inputs are seeded, identical from run to run for the same arguments.
 """
 import argparse
 import json
@@ -199,6 +202,42 @@ def run_reference_arm(args):
 # our arm
 # ---------------------------------------------------------------------------------------------
 
+DUMP_MAX_ROWS = 1_000_000   # 7 float64 columns: 56 MB at most
+
+
+def _mix64(x):
+    """splitmix64's finaliser on a uint64 array (wrapping arithmetic)."""
+    x = x ^ (x >> np.uint64(30))
+    x = x * np.uint64(0xbf58476d1ce4e5b9)
+    x = x ^ (x >> np.uint64(27))
+    x = x * np.uint64(0x94d049bb133111eb)
+    return x ^ (x >> np.uint64(31))
+
+
+def dump_outputs(rows, out_dir):
+    """The entries of a step (sorted by (table, k, seq)) as DIR/{table,k,seq,count}.npy in float64, every value exact:
+    seq is split into its four 32-bit words, least significant first (n x 4).  Above DUMP_MAX_ROWS entries the sample
+    is the DUMP_MAX_ROWS keys with the smallest seeded hash of (table, k, seq), still in table order: it depends on the
+    keys alone, so two builds whose tables differ in a few keys write samples that differ in about as few rows.
+    Returns what was written."""
+    n = int(rows.shape[0])
+    idx = np.arange(n)
+    if n > DUMP_MAX_ROWS:
+        meta = (rows["table"].astype(np.uint64) << np.uint64(8)) | rows["k"].astype(np.uint64)
+        with np.errstate(over="ignore"):
+            h = _mix64(_mix64(_mix64(meta ^ np.uint64(0x9e3779b97f4a7c15)) ^ rows["seq_lo"]) ^ rows["seq_hi"])
+        idx = np.sort(np.argpartition(h, DUMP_MAX_ROWS)[:DUMP_MAX_ROWS])
+    r = rows[idx]
+    mask = np.uint64(0xffffffff)
+    seq = np.stack([r["seq_lo"] & mask, r["seq_lo"] >> np.uint64(32), r["seq_hi"] & mask, r["seq_hi"] >> np.uint64(32)], axis=1)
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"table": r["table"], "k": r["k"], "seq": seq, "count": r["count"]}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
+    return {"dir": os.path.abspath(out_dir), "rows": n, "rows_written": int(idx.shape[0]),
+            "arrays": {name: list(a.shape) for name, a in arrays.items()}}
+
+
 def fastq_chunk(api, synth, seed, n_reads):
     """One raw chunk exactly as the reference's read_fastq_thread pushes it (QueueData, src/kmer.h:93-96): 4-line
     FASTQ text (header, sequence, '+', quality) plus the inclusive (st, nd) offsets of the sequence lines."""
@@ -290,6 +329,8 @@ def run_ours(args):
         sampler.window = (wall0, time.time())
         sampler.stop()
         table_rows = int(rows.shape[0])
+        # rows is a view of the library's entries: written out before the next step replaces them
+        dumped = dump_outputs(rows, args.dump_outputs) if args.dump_outputs else None
     # finish() and the merge run on the host between the event pair, so the event time covers the step
     ms = max_over_ranks(max(dev_ms, 0.0))
     wall_ms = max_over_ranks(wall_ms)
@@ -409,6 +450,8 @@ def run_ours(args):
             except Exception:
                 pass
         line.update(extra)
+        if dumped is not None:
+            line["outputs"] = dumped
         if world == 1 and not args.no_cpu_baseline:
             line["cpu_baseline"] = cpu_baseline()
         if world == 1 and not args.no_shapes:
@@ -559,7 +602,8 @@ def cpu_baseline():
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5,
+                    help="timed steps of the headline figure; the e2e and configs figures time min(steps, 5) steps each")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--reads", type=int, default=200_000_000, help="configs[1]: 200 M reads -- in total (strong) or per GPU (weak)")
@@ -570,7 +614,13 @@ def main():
     ap.add_argument("--full-tables", action="store_true", help="time the steps with every table row copied to the host (no report filter)")
     ap.add_argument("--no-weak", action="store_true", help="N > 1: skip the weak-scaling figure beside the strong one")
     ap.add_argument("--no-shapes", action="store_true", help="skip the paired / long / 3-64 shapes (configs[2..4])")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the tables of the last timed step to DIR/{table,k,seq,count}.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the tables of --impl ours")
     # stdout carries exactly one JSON line (rank 0): native libraries that print there (NCCL's version banner)
     # are diverted to stderr for the duration of the run
     sys.stdout.flush()

@@ -2,10 +2,13 @@
 without a usable GPU.  No GPU needed: every case ends before or at device-context creation."""
 import os
 import subprocess
+import sys
 
 import pytest
 
 from trew_b200 import api, synth
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def run(args):
@@ -60,14 +63,17 @@ def test_version_and_usage():
 
 
 def test_no_cpu_fallback(tmp_path):
-    """Without a usable CUDA device the program must fail loudly, never compute on the host."""
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("a GPU is present")
+    """Without a usable CUDA device the program must fail loudly, never compute on the host.  CUDA_VISIBLE_DEVICES=""
+    hides every device, so the check runs the same on a machine with a GPU and on one without."""
     p = os.path.join(str(tmp_path), "a.fastq")
     open(p, "wb").write(synth.fastq_bytes([b"TTAGGG" * 25]))
-    rc, out, err = run(["short", "5", "32", p])
-    assert rc == 1 and "cannot create device context" in err and out == ""
-    with pytest.raises(api.TrewError) as e:
-        api.DeviceContext(api.MODE_SHORT, 5, 32)
-    assert e.value.status == 2     # TREW_ERR_CUDA
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    r = subprocess.run([api.CLI_PATH, "short", "5", "32", p], capture_output=True, env=env)
+    assert r.returncode == 1 and b"cannot create device context" in r.stderr and r.stdout == b""
+    code = ("from trew_b200 import api\n"
+            "try:\n"
+            "    api.DeviceContext(api.MODE_SHORT, 5, 32)\n"
+            "except api.TrewError as e:\n"
+            "    print(e.status)\n")
+    r = subprocess.run([sys.executable, "-c", code], capture_output=True, env=env, cwd=ROOT)
+    assert r.stdout.decode().strip() == "2", r.stderr.decode()[-2000:]     # TREW_ERR_CUDA
