@@ -1818,8 +1818,10 @@ struct StageEmit {
 template <class K>
 constexpr size_t thread_kernel_smem() { return (size_t)et::Lay<K>::WORDS * TREW_THREAD_BLOCK * sizeof(u32) + (size_t)kStageSlots * 16; }
 constexpr size_t kThreadKernelSmem = thread_kernel_smem<et::u64>();
-// blocks per SM the kernels are built for: shared memory allows 6 (64-bit units: 61 words per thread + the staging table =
-// 35 KB) or 5 (128-bit units), the registers of the paired routing one less
+// blocks per SM the kernels are built for.  Shared memory would allow 8 (64-bit units: 47 words per thread + the staging
+// table = 27.5 KB, + 1 KB the driver reserves per block) or 6 (128-bit units, 59 words); the registers decide.  Short
+// reads, 64-bit units: 6 (80 registers); at 7 or 8 (72 / 64 registers) scan_window spills and the kernel is slower
+// (B200, 25 M-read batch: 0.589 / 0.613 / 0.641 ms at 6 / 7 / 8).  5 with 128-bit units, one less for the paired routing.
 template <int MODE, class K>
 constexpr int thread_kernel_bps() { return (sizeof(K) == 8 ? 6 : 5) - (MODE == 1 ? 1 : 0); }
 
