@@ -104,6 +104,7 @@ class Oracle:
         for name in ("orc_canon_c", "orc_crc_c"):
             getattr(L, name).argtypes = [C.c_uint64, C.c_uint64, C.c_int, C.POINTER(C.c_uint64)]
         L.orc_homo_c.argtypes = [C.c_uint64, C.c_uint64, C.c_int]
+        L.orc_period_stats.argtypes = [C.POINTER(_Cfg), C.c_char_p, C.c_int, C.c_int, C.c_int] + [C.c_void_p] * 5
 
     def scan(self, mode: int, reads1: Sequence[bytes], reads2: Optional[Sequence[bytes]] = None) -> Tables:
         t = self.lib.orc_tables_new()
@@ -130,6 +131,22 @@ class Oracle:
             return out[0], out[1], (sq[1] << 64) | sq[0], (sq[3] << 64) | sq[2], em
         finally:
             self.lib.orc_tables_free(t)
+
+    def period_stats(self, seq: bytes, st: int, nd: int, k: int) -> Tuple[int, int, int, int]:
+        """(T, M, S, n_classes) of period k over seq[st..nd] (inclusive): valid k-windows, the largest rotation class's
+        count, that class (the first to reach the maximum) and the number of classes."""
+        T, M, n = C.c_int(0), C.c_int(0), C.c_int(0)
+        lo, hi = C.c_uint64(0), C.c_uint64(0)
+        self.lib.orc_period_stats(C.byref(self.cfg), seq, st, nd, k, C.byref(T), C.byref(M), C.byref(lo), C.byref(hi), C.byref(n))
+        return T.value, M.value, (hi.value << 64) | lo.value, n.value
+
+    @staticmethod
+    def need(T: int, B: float) -> int:
+        """The smallest M with (double)M / T >= B (build_thr's threshold table); T + 1 when no M reaches it."""
+        M = max(0, int(B * T) - 2)
+        while M <= T and M / T < B:
+            M += 1
+        return M
 
     def canon(self, seq: int, k: int) -> int:
         o = (C.c_uint64 * 2)()
