@@ -209,8 +209,41 @@ int trew_dev_set_report_filter(trew_ctx* ctx, uint32_t min_total);
  * quarter full).  Call before merging other ranks' rows. */
 int trew_dev_reserve(trew_ctx* ctx, uint64_t expected_new_keys);
 
+/* ---- per-unit hit records: which unit put each count into the six tables ----------------------------------------------
+ *
+ * A unit is what the routing handles: one read (short and long mode) or one pair (paired mode).  A unit's records are the
+ * adds the reference's routing (buffer_task*) makes into the six final maps for that unit (the temp maps resolved), with
+ * adds to the same (table, k, seq) within the unit merged.  Summed over all units, the records give back the tables of
+ * trew_dev_finish (without the report filter, which records do not follow).
+ *
+ * The ordinal of a unit is its 0-based position among all units submitted to the context since create or reset, in call
+ * order, whatever the entry point: trew_dev_submit_chunk, trew_dev_submit_packed and trew_dev_scan_resident all count.
+ * trew_dev_process_file numbers the FASTQ records (pairs of records) of the file: after create or reset, the ordinal is the
+ * 0-based index of the record in the file (sequence line 4i + 2 for ordinal i).  Records the reader drops count too: in long
+ * mode the reads shorter than SLICE_LENGTH are kept and passed to the scan when records are on (they emit nothing, and
+ * trew_dev_get_stats counts them as reads).  Not supported on the one-process-per-GPU merge path (trew_dev_export_rows /
+ * trew_dev_merge_rows / trew_dev_finish_merged): merged rows have no unit. */
+typedef struct trew_unit_record { /* 32 bytes */
+    uint64_t unit;                  /* ordinal, see above                                                   */
+    uint64_t seq_lo, seq_hi;        /* the key exactly as added to the table (folded where the table is)    */
+    uint32_t count;
+    uint8_t table;                  /* TREW_TABLE_*                                                         */
+    uint8_t k;
+    uint16_t reserved;              /* 0                                                                    */
+} trew_unit_record;
+
+/* Record up to capacity_records records (32 bytes each, device memory) from now on; 0 switches recording off.  Only
+ * valid while the table is empty -- after create or reset -- TREW_ERR_ARG otherwise.  The appends keep counting past the
+ * capacity: nothing is lost silently (see trew_dev_unit_records), and the tables are not affected. */
+int trew_dev_enable_unit_records(trew_ctx* ctx, uint64_t capacity_records);
+/* Wait for all submitted work and return the records sorted by (unit, table, k, seq_hi, seq_lo), one row per key and
+ * unit.  The array (pinned host memory) belongs to the context and stays valid until the next call that touches the
+ * tables.  TREW_ERR_TABLE_FULL when more records were made than the capacity holds; trew_dev_last_error then names the
+ * capacity that would have been enough. */
+int trew_dev_unit_records(trew_ctx* ctx, const trew_unit_record** recs, uint64_t* n);
+
 /* Zero the count table (start of a new file; the reference allocates fresh maps per file,
- * src/kmer.cpp:89). */
+ * src/kmer.cpp:89).  Also clears the unit records and restarts the unit ordinals at 0. */
 int trew_dev_reset(trew_ctx* ctx);
 int trew_dev_get_stats(trew_ctx* ctx, trew_stats* out);
 
@@ -235,6 +268,12 @@ int trew_multi_reset(trew_multi* m);
 /* Drain every device, merge, return the six maps sorted by (table, k, seq) like trew_dev_finish (the array belongs to
  * the group and is valid until the next call that touches the tables). */
 int trew_multi_finish(trew_multi* m, const trew_entry** entries, uint64_t* n_entries);
+/* trew_dev_enable_unit_records / trew_dev_unit_records for the group.  The group assigns the ordinals in its own
+ * submission order (trew_multi_submit_chunk calls, across the round-robin dealing; trew_multi_process_file numbers
+ * the file's records as trew_dev_process_file does), and the devices' records are united on the first device.  trew_multi_reset
+ * clears them and restarts the ordinals at 0. */
+int trew_multi_enable_unit_records(trew_multi* m, uint64_t capacity_records);
+int trew_multi_unit_records(trew_multi* m, const trew_unit_record** recs, uint64_t* n);
 /* trew_dev_set_report_filter for the group's merged result. */
 int trew_multi_set_report_filter(trew_multi* m, uint32_t min_total);
 /* Sums over the group's contexts (device_ms: the largest). */

@@ -68,8 +68,27 @@ ABI_SYMBOLS = [
     "trew_pack_reads_ranges", "trew_report_text", "trew_synth_resident_ex", "trew_multi_create", "trew_multi_destroy",
     "trew_multi_device_count", "trew_multi_last_error", "trew_multi_submit_chunk", "trew_multi_process_file",
     "trew_multi_reset", "trew_multi_finish", "trew_multi_get_stats", "trew_multi_ctx", "trew_dev_set_report_filter",
-    "trew_multi_set_report_filter",
+    "trew_multi_set_report_filter", "trew_dev_enable_unit_records", "trew_dev_unit_records", "trew_multi_enable_unit_records",
+    "trew_multi_unit_records",
 ]
+
+# trew_unit_record: one unit's adds to one (table, k, seq), sorted by (unit, table, k, seq_hi, seq_lo)
+UNIT_RECORD_DTYPE = np.dtype([("unit", "<u8"), ("seq_lo", "<u8"), ("seq_hi", "<u8"), ("count", "<u4"), ("table", "u1"),
+                              ("k", "u1"), ("reserved", "<u2")])
+UnitRecords = Dict[Tuple[int, int, int, int], int]
+
+
+def unit_records_dict(recs: np.ndarray) -> UnitRecords:
+    """A unit_records() array as {(unit, table, k, seq): count}."""
+    return {(int(r["unit"]), int(r["table"]), int(r["k"]), (int(r["seq_hi"]) << 64) | int(r["seq_lo"])): int(r["count"])
+            for r in recs}
+
+
+def _records_array(p: C.c_void_p, n: int) -> np.ndarray:
+    if n == 0:
+        return np.zeros(0, dtype=UNIT_RECORD_DTYPE)
+    buf = (C.c_char * (n * UNIT_RECORD_DTYPE.itemsize)).from_address(p.value)
+    return np.frombuffer(buf, dtype=UNIT_RECORD_DTYPE, count=n).copy()
 
 CHUNK_SINK = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.POINTER(C.c_int32), C.c_uint32, C.c_void_p,
                         C.POINTER(C.c_int32), C.c_uint32)
@@ -134,6 +153,10 @@ def load_library() -> C.CDLL:
     L.trew_multi_ctx.restype = C.c_void_p
     L.trew_dev_set_report_filter.argtypes = [C.c_void_p, C.c_uint32]
     L.trew_multi_set_report_filter.argtypes = [C.c_void_p, C.c_uint32]
+    L.trew_dev_enable_unit_records.argtypes = [C.c_void_p, C.c_uint64]
+    L.trew_dev_unit_records.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64)]
+    L.trew_multi_enable_unit_records.argtypes = [C.c_void_p, C.c_uint64]
+    L.trew_multi_unit_records.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64)]
     L.trew_dev_timer_start.argtypes = [C.c_void_p]
     L.trew_dev_timer_stop.argtypes = [C.c_void_p, C.POINTER(C.c_float)]
     L.trew_dev_kernel_times.argtypes = [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_double),
@@ -409,6 +432,17 @@ class DeviceContext:
     def reset(self) -> None:
         self._check(self.lib.trew_dev_reset(self.ctx))
 
+    def enable_unit_records(self, capacity: int) -> None:
+        """Record which unit (read, or pair in paired mode) made each table add, for up to `capacity` records; 0 = off.
+        Only while the table is empty (after create or reset)."""
+        self._check(self.lib.trew_dev_enable_unit_records(self.ctx, capacity))
+
+    def unit_records(self) -> np.ndarray:
+        """The records so far as a structured array (UNIT_RECORD_DTYPE), sorted by (unit, table, k, seq); a copy."""
+        p, n = C.c_void_p(), C.c_uint64()
+        self._check(self.lib.trew_dev_unit_records(self.ctx, C.byref(p), C.byref(n)))
+        return _records_array(p, n.value)
+
     def stats(self) -> Stats:
         s = Stats()
         self._check(self.lib.trew_dev_get_stats(self.ctx, C.byref(s)))
@@ -492,6 +526,16 @@ class MultiContext:
 
     def reset(self) -> None:
         self._check(self.lib.trew_multi_reset(self.h))
+
+    def enable_unit_records(self, capacity: int) -> None:
+        """DeviceContext.enable_unit_records for every device of the group (capacity per device)."""
+        self._check(self.lib.trew_multi_enable_unit_records(self.h, capacity))
+
+    def unit_records(self) -> np.ndarray:
+        """The group's records (ordinals in its submission order), united on the first device; a copy."""
+        p, n = C.c_void_p(), C.c_uint64()
+        self._check(self.lib.trew_multi_unit_records(self.h, C.byref(p), C.byref(n)))
+        return _records_array(p, n.value)
 
     def finish_view(self) -> np.ndarray:
         p = C.POINTER(Entry)()

@@ -102,6 +102,13 @@ struct trew_ctx {
     void* h_export = nullptr; size_t h_export_bytes = 0;
     unsigned int report_min = 0;                                 // > 0: finish copies only the rows a one-file report can show
     trew_entry* d_filtered = nullptr; size_t d_filtered_cap = 0;
+    // unit records (trew_dev_enable_unit_records): dcfg.recs points at d_recs when they are on
+    UnitRecs* d_recs = nullptr; trew_unit_record* d_rec_buf = nullptr; uint64_t rec_cap = 0;
+    uint64_t unit_next = 0;                      // ordinal of the next unit submitted
+    bool table_used = false;                     // something was scanned or merged since create / reset
+    trew_unit_record* d_rec_out = nullptr; size_t d_rec_out_cap = 0;   // sorted, combined records
+    trew_unit_record* d_rec_cat = nullptr; size_t d_rec_cat_cap = 0;   // trew_multi: every device's records on the first one
+    void* h_rec = nullptr; size_t h_rec_bytes = 0;
 };
 
 namespace {
@@ -183,11 +190,15 @@ int launch_scan(trew_ctx* ctx, const DevBatch& b, uint32_t n_units, uint32_t max
         *scratch_bytes = need;
     }
     ctx->export_valid = false;
+    ctx->table_used = true;
+    DevCfg cfg = ctx->dcfg;
+    cfg.unit_base = ctx->unit_next;
+    ctx->unit_next += n_units;
     // d_counters: [0] survivors (list A) [1] work counter [2] deferred [3] thread-kernel bails [4] survivors, list B [5] work counter [6] work counter of the thread kernel [7] work counter of the decide kernel
     CK(cudaMemsetAsync(d_counters, 0, kScanCounters * sizeof(unsigned int), st));
     if (ev) CK(cudaEventRecord(ev[0], st));
-    const bool thread_path = thread_path_applies(ctx->dcfg, max_read_len) && !(ctx->exact_flags & 4u) && n_units < (1u << 28);
-    launch_filter(ctx->dcfg, b, n_units, max_read_len, d_survivors + n_units, d_counters + 2, d_survivors, d_counters, ctx->plan, st,
+    const bool thread_path = thread_path_applies(cfg, max_read_len) && !(ctx->exact_flags & 4u) && n_units < (1u << 28);
+    launch_filter(cfg, b, n_units, max_read_len, d_survivors + n_units, d_counters + 2, d_survivors, d_counters, ctx->plan, st,
                   ev ? ev[1] : nullptr, thread_path ? d_survivors + n_units - 1 : nullptr, thread_path ? d_counters + 4 : nullptr,
                   d_counters + 7);
     if (ev) CK(cudaEventRecord(ev[2], st));
@@ -200,12 +211,12 @@ int launch_scan(trew_ctx* ctx, const DevBatch& b, uint32_t n_units, uint32_t max
     if (thread_path) {
         // list A: thread per survivor; what it cannot take after all (its length limits) lands in the dead deferred list
         unsigned int* hard = d_survivors + n_units;
-        launch_exact_thread(ctx->dcfg, b, d_survivors, d_counters, a.packed_probes, hard, d_counters + 3, ctx->d_total_surv,
+        launch_exact_thread(cfg, b, d_survivors, d_counters, a.packed_probes, hard, d_counters + 3, ctx->d_total_surv,
                             ctx->sm_count, env_blocks_thread(), d_counters + 6, st);
         // list B (downwards from the top of the survivor array): warp per survivor
         ExactArgs ab = a;
         ab.survivors = d_survivors + n_units - 1; ab.reverse = 1; ab.n_survivors = d_counters + 4;
-        launch_exact(ctx->dcfg, b, ab, ctx->plan, st);
+        launch_exact(cfg, b, ab, ctx->plan, st);
         // ... and the thread kernel's leftovers (normally none)
         a.survivors = hard; a.n_survivors = d_counters + 3; a.work_counter = d_counters + 5; a.total_survivors = nullptr;
         ctx->stats.kernel_launches += 2;
@@ -213,12 +224,12 @@ int launch_scan(trew_ctx* ctx, const DevBatch& b, uint32_t n_units, uint32_t max
         // long reads: statistics of every slice of a survivor, the walks over them, the emissions (three kernels); reads
         // whose walk reaches the long middle slice -- or beyond the scratch's capacity -- go to the warp kernel
         unsigned int* hard = d_survivors + n_units;
-        launch_long_thread(ctx->dcfg, b, d_survivors, d_counters, a.packed_probes, s_cap, max_slices, *d_scratch + long_off, hard,
+        launch_long_thread(cfg, b, d_survivors, d_counters, a.packed_probes, s_cap, max_slices, *d_scratch + long_off, hard,
                            d_counters + 3, ctx->d_total_surv, ctx->sm_count, st);
         a.survivors = hard; a.n_survivors = d_counters + 3; a.total_survivors = nullptr;
         ctx->stats.kernel_launches += 3;
     }
-    launch_exact(ctx->dcfg, b, a, ctx->plan, st);
+    launch_exact(cfg, b, a, ctx->plan, st);
     if (ev) CK(cudaEventRecord(ev[3], st));
     CK(cudaGetLastError());
     ctx->stats.kernel_launches += 3;
@@ -484,6 +495,11 @@ int fork_aux(trew_ctx* ctx) {
     return TREW_OK;
 }
 
+// Long mode: the reader drops reads shorter than SLICE_LENGTH (src/kmer.cpp:1184).  With unit records on it keeps them, so
+// that unit ordinals are the file's record indices; the scan emits nothing for them (unit_probes, route_long), so the tables
+// are the same.
+int reader_slice_length(const trew_ctx* ctx) { return ctx->d_recs ? 0 : ctx->cfg.slice_length; }
+
 int check_device_error(trew_ctx* ctx) {
     unsigned int e = 0;
     CK(cudaMemcpy(&e, ctx->d_error, sizeof(e), cudaMemcpyDeviceToHost));
@@ -668,6 +684,11 @@ void trew_dev_destroy(trew_ctx* ctx) {
     if (ctx->d_sort_tmp) cudaFree(ctx->d_sort_tmp);
     if (ctx->d_n) cudaFree(ctx->d_n);
     if (ctx->h_export) cudaFreeHost(ctx->h_export);
+    if (ctx->d_recs) cudaFree(ctx->d_recs);
+    if (ctx->d_rec_buf) cudaFree(ctx->d_rec_buf);
+    if (ctx->d_rec_out) cudaFree(ctx->d_rec_out);
+    if (ctx->d_rec_cat) cudaFree(ctx->d_rec_cat);
+    if (ctx->h_rec) cudaFreeHost(ctx->h_rec);
     if (ctx->main_stream) cudaStreamDestroy(ctx->main_stream);
     if (ctx->aux_stream) cudaStreamDestroy(ctx->aux_stream);
     if (ctx->ev_join) cudaEventDestroy(ctx->ev_join);
@@ -961,6 +982,57 @@ int finish_rows(trew_ctx* ctx, const trew_entry* d_in, uint64_t n_in, bool combi
     return rows_to_host(ctx, rows, n, entries, n_entries);
 }
 
+// records made so far on ctx (synchronised); TREW_ERR_TABLE_FULL when they did not fit its capacity
+int unit_record_count(trew_ctx* ctx, uint64_t* made) {
+    unsigned long long m = 0;
+    CK(cudaMemcpy(&m, &ctx->d_recs->n, sizeof(m), cudaMemcpyDeviceToHost));
+    *made = m;
+    if (m > ctx->rec_cap)
+        return fail(ctx, TREW_ERR_TABLE_FULL, "unit records overflowed: %llu records made, capacity %llu (a capacity of %llu is enough)", m,
+                    (unsigned long long)ctx->rec_cap, m);
+    return TREW_OK;
+}
+
+// n unit records in ctx's device memory -> sorted by (unit, table, k, seq), equal keys summed -> the pinned host array
+int records_to_host(trew_ctx* ctx, const trew_unit_record* d_in, uint64_t n_in, const trew_unit_record** recs, uint64_t* n_out) {
+    if (n_in > 0x7fffffffULL) return fail(ctx, TREW_ERR_ARG, "too many unit records (%llu)", (unsigned long long)n_in);
+    if (n_in > ctx->d_rec_out_cap) {
+        if (ctx->d_rec_out) CK(cudaFree(ctx->d_rec_out));
+        ctx->d_rec_out = nullptr;
+        ctx->d_rec_out_cap = (size_t)n_in + n_in / 4 + 1024;
+        CK(cudaMalloc((void**)&ctx->d_rec_out, ctx->d_rec_out_cap * sizeof(trew_unit_record)));
+    }
+    const unsigned int n = (unsigned int)n_in;
+    const bool wide = ctx->cfg.max_mer > 32;
+    size_t need = 0;
+    CK(sort_combine_records(d_in, n, wide, ctx->d_rec_out, ctx->d_n, nullptr, &need, ctx->main_stream));
+    if (need > ctx->sort_tmp_bytes) {
+        CK(cudaStreamSynchronize(ctx->main_stream));
+        if (ctx->d_sort_tmp) CK(cudaFree(ctx->d_sort_tmp));
+        ctx->d_sort_tmp = nullptr;
+        ctx->sort_tmp_bytes = need + need / 4;
+        CK(cudaMalloc(&ctx->d_sort_tmp, ctx->sort_tmp_bytes));
+    }
+    size_t bytes = ctx->sort_tmp_bytes;
+    CK(sort_combine_records(d_in, n, wide, ctx->d_rec_out, ctx->d_n, ctx->d_sort_tmp, &bytes, ctx->main_stream));
+    unsigned int m = 0;
+    CK(cudaMemcpyAsync(&m, ctx->d_n, sizeof(m), cudaMemcpyDeviceToHost, ctx->main_stream));
+    CK(cudaStreamSynchronize(ctx->main_stream));
+    const size_t need_host = (size_t)m * sizeof(trew_unit_record) + 64;
+    if (need_host > ctx->h_rec_bytes) {
+        if (ctx->h_rec) CK(cudaFreeHost(ctx->h_rec));
+        ctx->h_rec = nullptr;
+        const size_t cap = std::max(need_host + need_host / 2, (size_t)1 << 20);
+        CK(cudaHostAlloc(&ctx->h_rec, cap, cudaHostAllocDefault));
+        ctx->h_rec_bytes = cap;
+    }
+    if (m) CK(cudaMemcpy(ctx->h_rec, ctx->d_rec_out, (size_t)m * sizeof(trew_unit_record), cudaMemcpyDeviceToHost));
+    ctx->stats.d2h_bytes += (uint64_t)m * sizeof(trew_unit_record) + 4;
+    *recs = (const trew_unit_record*)ctx->h_rec;
+    *n_out = m;
+    return TREW_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1033,6 +1105,7 @@ int trew_dev_merge_rows(trew_ctx* ctx, const trew_entry* d_rows, uint64_t n_rows
     if (!ctx || (n_rows && !d_rows) || n_rows > 0xffffffffULL) return TREW_ERR_ARG;
     CK(cudaSetDevice(ctx->cfg.device));
     ctx->export_valid = false;
+    ctx->table_used = true;
     ctx->keys_seen = std::max<unsigned int>(ctx->keys_seen, (unsigned int)(ctx->n_slots / 16 + 1));
     launch_merge_entries(ctx->dcfg, d_rows, (unsigned int)n_rows, ctx->main_stream);   // asynchronous: the next sync / export
     CK(cudaGetLastError());                                                             // waits and checks the error flag
@@ -1065,10 +1138,42 @@ int trew_dev_reset(trew_ctx* ctx) {
     // on the scan stream (the context's streams do not synchronise with the legacy default stream)
     CK(cudaMemsetAsync(ctx->dcfg.slots, 0, ctx->n_slots * sizeof(Slot), ctx->main_stream));
     CK(cudaMemsetAsync(ctx->d_error, 0, 2 * sizeof(unsigned int), ctx->main_stream));
+    if (ctx->d_recs) CK(cudaMemsetAsync(&ctx->d_recs->n, 0, sizeof(unsigned long long), ctx->main_stream));
     CK(cudaStreamSynchronize(ctx->main_stream));
+    ctx->unit_next = 0;
+    ctx->table_used = false;
     ctx->keys_seen = 0;
     for (auto& sl : ctx->slots) *sl.h_keys = 0;
     return TREW_OK;
+}
+
+int trew_dev_enable_unit_records(trew_ctx* ctx, uint64_t capacity_records) {
+    if (!ctx) return TREW_ERR_ARG;
+    if (ctx->table_used) return fail(ctx, TREW_ERR_ARG, "unit records can only be switched on or off while the table is empty (after create or reset)");
+    if (capacity_records > 0x7fffffffULL) return fail(ctx, TREW_ERR_ARG, "unit record capacity above 2^31 - 1");
+    CK(cudaSetDevice(ctx->cfg.device));
+    CK(cudaStreamSynchronize(ctx->main_stream));
+    if (ctx->d_rec_buf) CK(cudaFree(ctx->d_rec_buf));
+    if (ctx->d_recs) CK(cudaFree(ctx->d_recs));
+    ctx->d_rec_buf = nullptr; ctx->d_recs = nullptr; ctx->dcfg.recs = nullptr; ctx->rec_cap = 0;
+    if (capacity_records == 0) return TREW_OK;
+    CK(cudaMalloc((void**)&ctx->d_rec_buf, capacity_records * sizeof(trew_unit_record)));
+    CK(cudaMalloc((void**)&ctx->d_recs, sizeof(UnitRecs)));
+    const UnitRecs r{ctx->d_rec_buf, (unsigned long long)capacity_records, 0ULL};
+    CK(cudaMemcpy(ctx->d_recs, &r, sizeof(r), cudaMemcpyHostToDevice));
+    ctx->rec_cap = capacity_records;
+    ctx->dcfg.recs = ctx->d_recs;
+    return TREW_OK;
+}
+
+int trew_dev_unit_records(trew_ctx* ctx, const trew_unit_record** recs, uint64_t* n) {
+    if (!ctx || !recs || !n) return TREW_ERR_ARG;
+    if (!ctx->d_recs) return fail(ctx, TREW_ERR_ARG, "unit records are off (trew_dev_enable_unit_records)");
+    int rc = trew_dev_sync(ctx);
+    if (rc) return rc;
+    uint64_t made = 0;
+    if ((rc = unit_record_count(ctx, &made)) != TREW_OK) return rc;
+    return records_to_host(ctx, ctx->d_rec_buf, made, recs, n);
 }
 
 int trew_dev_get_stats(trew_ctx* ctx, trew_stats* out) {
@@ -1155,7 +1260,7 @@ int trew_dev_process_file(trew_ctx* ctx, const char* file1, int is_gz1, const ch
     if ((ctx->cfg.mode == TREW_MODE_PAIR) != (file2 != nullptr)) return fail(ctx, TREW_ERR_ARG, "second file only in pair mode");
     // plain files: large blocks read and indexed by the pool; .gz: the inflate stream is sequential, keep blocks small
     const size_t chunk = 0;   // the reader picks the block size by input kind
-    IngestResult r = ingest_file(ctx->cfg.mode, ctx->cfg.slice_length, file1, is_gz1 != 0, file2, is_gz2 != 0, chunk,
+    IngestResult r = ingest_file(ctx->cfg.mode, reader_slice_length(ctx), file1, is_gz1 != 0, file2, is_gz2 != 0, chunk,
                                  [&](const char* b1, const std::vector<int32_t>& l1, const char* b2, const std::vector<int32_t>& l2) {
                                      return trew_dev_submit_chunk(ctx, b1, l1.data(), (uint32_t)(l1.size() / 2), b2,
                                                                   b2 ? l2.data() : nullptr, b2 ? (uint32_t)(l2.size() / 2) : 0u);
@@ -1175,6 +1280,7 @@ struct trew_multi {
     std::vector<trew_ctx*> ctx;
     Pool* pool = nullptr;
     size_t next = 0;                  // device the next chunk goes to
+    uint64_t unit_next = 0;           // unit ordinal of the group's next submitted unit
     std::string err;
     // per peer device: its rows as copied to the first device (device-0 memory)
     std::vector<trew_entry*> d_peer; std::vector<size_t> d_peer_cap;
@@ -1182,6 +1288,8 @@ struct trew_multi {
 
 namespace {
 int mfail(trew_multi* m, int status, const std::string& msg) { if (m) m->err = msg; return status; }
+// units of one submitted chunk (index-wise pairing in paired mode, src/kmer.cpp:321-322)
+uint64_t chunk_units(const trew_ctx* x, uint32_t n1, uint32_t n2) { return x->cfg.mode == TREW_MODE_PAIR ? std::min(n1, n2) : n1; }
 }  // namespace
 
 extern "C" {
@@ -1258,8 +1366,10 @@ int trew_multi_submit_chunk(trew_multi* m, const char* buffer1, const int32_t* l
     if (!m) return TREW_ERR_ARG;
     trew_ctx* x = m->ctx[m->next];
     m->next = (m->next + 1) % m->ctx.size();
+    x->unit_next = m->unit_next;   // the group's submission order
     int rc = trew_dev_submit_chunk(x, buffer1, locs1, n1, buffer2, locs2, n2);
     if (rc != TREW_OK) return mfail(m, rc, x->err);
+    m->unit_next += chunk_units(x, n1, n2);
     return TREW_OK;
 }
 
@@ -1268,7 +1378,7 @@ int trew_multi_process_file(trew_multi* m, const char* file1, int is_gz1, const 
     trew_ctx* x0 = m->ctx[0];
     if ((x0->cfg.mode == TREW_MODE_PAIR) != (file2 != nullptr)) return mfail(m, TREW_ERR_ARG, "second file only in pair mode");
     // one reader, N consumers: every block of the file goes to the next device
-    IngestResult r = ingest_file(x0->cfg.mode, x0->cfg.slice_length, file1, is_gz1 != 0, file2, is_gz2 != 0, 0,
+    IngestResult r = ingest_file(x0->cfg.mode, reader_slice_length(x0), file1, is_gz1 != 0, file2, is_gz2 != 0, 0,
                                  [&](const char* b1, const std::vector<int32_t>& l1, const char* b2, const std::vector<int32_t>& l2) {
                                      return trew_multi_submit_chunk(m, b1, l1.data(), (uint32_t)(l1.size() / 2), b2, b2 ? l2.data() : nullptr,
                                                                     b2 ? (uint32_t)(l2.size() / 2) : 0u);
@@ -1282,6 +1392,7 @@ int trew_multi_reset(trew_multi* m) {
     if (!m) return TREW_ERR_ARG;
     for (trew_ctx* x : m->ctx) { int rc = trew_dev_reset(x); if (rc != TREW_OK) return mfail(m, rc, x->err); }
     m->next = 0;
+    m->unit_next = 0;
     return TREW_OK;
 }
 
@@ -1319,6 +1430,58 @@ int trew_multi_finish(trew_multi* m, const trew_entry** entries, uint64_t* n_ent
         sizes.push_back(n_rows[i]);
     }
     int rc = trew_dev_finish_merged(x0, lists.data(), sizes.data(), (uint32_t)lists.size(), entries, n_entries);
+    return rc == TREW_OK ? rc : mfail(m, rc, x0->err);
+}
+
+int trew_multi_enable_unit_records(trew_multi* m, uint64_t capacity_records) {
+    if (!m) return TREW_ERR_ARG;
+    for (trew_ctx* x : m->ctx) {
+        int rc = trew_dev_enable_unit_records(x, capacity_records);
+        if (rc != TREW_OK) return mfail(m, rc, x->err);
+    }
+    return TREW_OK;
+}
+
+int trew_multi_unit_records(trew_multi* m, const trew_unit_record** recs, uint64_t* n) {
+    if (!m || !recs || !n) return TREW_ERR_ARG;
+    trew_ctx* x0 = m->ctx[0];
+    if (!x0->d_recs) return mfail(m, TREW_ERR_ARG, "unit records are off (trew_multi_enable_unit_records)");
+    const size_t nd = m->ctx.size();
+    std::vector<uint64_t> made(nd, 0);
+    uint64_t total = 0, most = 0;
+    int full = TREW_OK;
+    for (size_t i = 0; i < nd; i++) {
+        int rc = trew_dev_sync(m->ctx[i]);   // a count-table overflow is reported as such
+        if (rc != TREW_OK) return mfail(m, rc, m->ctx[i]->err);
+        rc = unit_record_count(m->ctx[i], &made[i]);
+        if (rc == TREW_ERR_TABLE_FULL) full = rc;
+        else if (rc != TREW_OK) return mfail(m, rc, m->ctx[i]->err);
+        total += made[i]; most = std::max(most, made[i]);
+    }
+    if (full != TREW_OK)
+        return mfail(m, full, "unit records overflowed on a device: " + std::to_string(most) + " records made, capacity " +
+                                  std::to_string(x0->rec_cap) + " (a capacity of " + std::to_string(most) + " is enough)");
+    if (nd == 1) {
+        int rc = records_to_host(x0, x0->d_rec_buf, made[0], recs, n);
+        return rc == TREW_OK ? rc : mfail(m, rc, x0->err);
+    }
+    // every device's records to the first device (units are disjoint across devices), then one sort
+    trew_ctx* ctx = x0;   // for CK
+    CK(cudaSetDevice(x0->cfg.device));
+    if (total > x0->d_rec_cat_cap) {
+        if (x0->d_rec_cat) CK(cudaFree(x0->d_rec_cat));
+        x0->d_rec_cat = nullptr;
+        x0->d_rec_cat_cap = (size_t)total + total / 4 + 1024;
+        CK(cudaMalloc((void**)&x0->d_rec_cat, x0->d_rec_cat_cap * sizeof(trew_unit_record)));
+    }
+    uint64_t at = 0;
+    for (size_t i = 0; i < nd; i++) {
+        if (made[i])
+            CK(cudaMemcpyPeerAsync(x0->d_rec_cat + at, x0->cfg.device, m->ctx[i]->d_rec_buf, m->ctx[i]->cfg.device,
+                                   made[i] * sizeof(trew_unit_record), x0->main_stream));
+        at += made[i];
+    }
+    int rc = records_to_host(x0, x0->d_rec_cat, total, recs, n);
     return rc == TREW_OK ? rc : mfail(m, rc, x0->err);
 }
 

@@ -102,6 +102,23 @@ __device__ __noinline__ void table_add_impl(Slot* slots, u32 slot_mask, u32* err
     atomicExch(error_flag, 3u);  // TREW_ERR_TABLE_FULL
 }
 
+// one unit record per calling thread.  Space is reserved once for the threads of the warp that arrive together (the
+// routing emits the same few keys from every survivor, and same-address atomics retire one at a time in L2); the counter
+// keeps counting past the capacity so that the host can tell how much would have been enough.
+__device__ __forceinline__ void rec_append(UnitRecs* R, u64 unit, int table, int k, u64 lo, u64 hi, u64 count) {
+    const u32 act = __activemask(), lane = threadIdx.x & 31;
+    const int leader = __ffs(act) - 1;
+    u64 base = 0;
+    if ((int)lane == leader) base = atomicAdd(&R->n, (u64)__popc(act));
+    base = __shfl_sync(act, base, leader);
+    const u64 i = base + (u64)__popc(act & ((1u << lane) - 1u));
+    if (i < R->cap) {
+        uint4* p = reinterpret_cast<uint4*>(R->buf + i);
+        p[0] = make_uint4((u32)unit, (u32)(unit >> 32), (u32)lo, (u32)(lo >> 32));
+        p[1] = make_uint4((u32)hi, (u32)(hi >> 32), (u32)count, (u32)table | ((u32)k << 8));
+    }
+}
+
 // adds another table's entries to this one: the device-side analogue of the per-thread map sum, src/kmer.cpp:1486-1515
 __global__ void merge_entries_kernel(Slot* slots, u32 slot_mask, u32* error_flag, const trew_entry* __restrict__ e, u32 n) {
     for (u32 i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
@@ -895,9 +912,11 @@ constexpr int kSerialMaxRuns = 12;   // eval_k: windows with at most this many m
 
 // header words.  12..27: the state of one scan_stats() call -- warp-uniform, so it lives here once instead of in
 // every lane's registers (which the calls into eval_k would spill to local memory)
-enum { HD_CUR_POS = 0, HD_CUR_LEN, HD_ALLVALID, HD_EV_POS, HD_EV_LEN, HD_EV_K, HD_EV_PACK, HD_S = 8 /* 4 words: s_lo, s_hi */,
+enum { HD_CUR_POS = 0, HD_CUR_LEN, HD_ALLVALID, HD_EV_POS, HD_EV_LEN, HD_EV_K, HD_EV_PACK, HD_UNIT = 7 /* the survivor's unit index in the batch */,
+       HD_S = 8 /* 4 words: s_lo, s_hi */,
        HD_BLK_L = 12 /* 2 words */, HD_BLK_H = 14 /* 2 words */, HD_NEED_L = 16, HD_NEED_H = 17, HD_BLK64 = 18, HD_RES = 19,
-       HD_SH = 20 /* 4 words */, HD_SL = 24 /* 4 words */ };
+       HD_SH = 20 /* 4 words */, HD_SL = 24 /* 4 words */, HD_UNIT_BASE = 28 /* 2 words: ordinal of the batch's unit 0 */,
+       HD_RECS = 30 /* 2 words: UnitRecs*, 0 = no records */ };
 constexpr int kHeaderBytes = 128;
 
 __host__ __device__ inline int exact_hash_slots(int cap) {
@@ -1333,7 +1352,9 @@ __device__ __forceinline__ void eval_S(WS ws, u64& lo, u64& hi) {
     hi = (u64)hd[HD_S + 2] | ((u64)hd[HD_S + 3] << 32);
 }
 
-// add every distinct class of the last eval_k() to a result table (optionally RC-folded)
+// add every distinct class of the last eval_k() to a result table (optionally RC-folded); REC: and record them for the
+// survivor's unit (the kernel's instantiation with records)
+template <bool REC>
 __device__ __noinline__ void emit_classes(TableRef tr, WS ws, int k, int nruns, int table, bool folded) {
     u32 meta = ((u32)table << 8) | (u32)k;
     const unsigned short* run_total = ws.run_total();
@@ -1348,6 +1369,11 @@ __device__ __noinline__ void emit_classes(TableRef tr, WS ws, int k, int nruns, 
             if (less_pair(rlo, rhi, lo, hi)) { lo = rlo; hi = rhi; }
         }
         table_add_impl(tr.slots, tr.mask, tr.err, meta, lo, hi, (u64)total);
+        if constexpr (REC) {
+            const u32* hd = ws.hdr();
+            UnitRecs* R = reinterpret_cast<UnitRecs*>((u64)hd[HD_RECS] | ((u64)hd[HD_RECS + 1] << 32));
+            rec_append(R, ((u64)hd[HD_UNIT_BASE] | ((u64)hd[HD_UNIT_BASE + 1] << 32)) + hd[HD_UNIT], table, k, lo, hi, (u64)total);
+        }
     }
     __syncwarp();
 }
@@ -1555,15 +1581,17 @@ __device__ __noinline__ u32 eval_cached(WS ws, DevBatch b, u32 pos, int len, int
 }
 
 // the emission half of k_mer_check for one target k (src/kmer.cpp:2264-2328): every class, un-folded unless asked
+template <bool REC>
 __device__ void emit_window(TableRef tr, WS ws, const DevBatch& b, u32 pos, int len, int k, int table, bool folded) {
     u32 ev = eval_cached(ws, b, pos, len, k);
-    emit_classes(tr, ws, k, pk_runs(ev), table, folded);
+    emit_classes<REC>(tr, ws, k, pk_runs(ev), table, folded);
 }
 
 // k_mer_target / k_mer_target_128 (src/kmer.cpp:1894-2142)
+template <bool REC>
 __device__ void target_window(TableRef tr, WS ws, const DevBatch& b, u32 pos, int len, int k, const unsigned short* thr_low, bool high, int table) {
     u32 ev = eval_cached(ws, b, pos, len, k);
-    if (pk_T(ev) > 0 && !pk_homo(ev) && pk_M(ev) >= thr_at(ws, thr_low, high, pk_T(ev))) emit_classes(tr, ws, k, pk_runs(ev), table, true);
+    if (pk_T(ev) > 0 && !pk_homo(ev) && pk_M(ev) >= thr_at(ws, thr_low, high, pk_T(ev))) emit_classes<REC>(tr, ws, k, pk_runs(ev), table, true);
 }
 
 // ---- routing -----------------------------------------------------------------------------------
@@ -1572,6 +1600,7 @@ enum { T_F = 0, T_B = 2, T_O = 4 };
 
 // buffer_task (src/kmer.cpp:80-266)
 // pm: probes (unit_probes order) the filter kernels could not rule out; the scan of any other window finds nothing
+template <bool REC>
 __device__ void route_short(const DevCfg& cfg, TableRef tr, WS ws, const DevBatch& b, u32 u, u32 pm) {
     const int MINM = cfg.min_mer, MAXM = cfg.max_mer;
     u32 b0 = __ldg(b.bit_off + u);
@@ -1589,21 +1618,22 @@ __device__ void route_short(const DevCfg& cfg, TableRef tr, WS ws, const DevBatc
         // (nullptr maps at src/kmer.cpp:125, result.backward at :158)
 #pragma unroll
         for (int c = 0; c < 2; c++) {
-            if (L[c] > 0 && L[c] == R[c]) target_window(tr, ws, b, b0, n, L[c], cfg.thr_low, c == 0, T_O + c);
-            else if (L[c] > 0) emit_window(tr, ws, b, lpos, llen, L[c], T_F + c, false);
-            else if (R[c] > 0) emit_window(tr, ws, b, rpos, rlen, R[c], T_B + c, false);
+            if (L[c] > 0 && L[c] == R[c]) target_window<REC>(tr, ws, b, b0, n, L[c], cfg.thr_low, c == 0, T_O + c);
+            else if (L[c] > 0) emit_window<REC>(tr, ws, b, lpos, llen, L[c], T_F + c, false);
+            else if (R[c] > 0) emit_window<REC>(tr, ws, b, rpos, rlen, R[c], T_B + c, false);
         }
     }
     bool hc[2] = {L[0] == 0 && R[0] == 0, L[1] == 0 && R[1] == 0};
     if (4 * MAXM > n && (hc[0] || hc[1]) && (pm & 1u)) {
         ScanRes s = scan_stats(ws, b, b0, n, max(n / 4 + 1, MINM), min(n / 2, MAXM), cfg);
-        if (hc[0] && s.th) emit_window(tr, ws, b, b0, n, s.th, T_O + 0, false);  // un-folded into 'both'
-        if (hc[1] && s.tl) emit_window(tr, ws, b, b0, n, s.tl, T_O + 1, false);
+        if (hc[0] && s.th) emit_window<REC>(tr, ws, b, b0, n, s.th, T_O + 0, false);  // un-folded into 'both'
+        if (hc[1] && s.tl) emit_window<REC>(tr, ws, b, b0, n, s.tl, T_O + 1, false);
     }
 }
 
 // buffer_task_pair (src/kmer.cpp:268-745); follows the 128-bit path where the two differ (temp map cleared
 // after the large-k block, src/kmer.cpp:722-723)
+template <bool REC>
 __device__ void route_pair(const DevCfg& cfg, TableRef tr, WS ws, const DevBatch& b, u32 u) {
     const int MINM = cfg.min_mer, MAXM = cfg.max_mer;
     u32 a0 = __ldg(b.bit_off + 2 * u), a1 = __ldg(b.bit_off + 2 * u + 1), a2 = __ldg(b.bit_off + 2 * u + 2);
@@ -1643,7 +1673,7 @@ __device__ void route_pair(const DevCfg& cfg, TableRef tr, WS ws, const DevBatch
             if (si[c] == 5) {
                 for (int e = 0; e < np[c]; e++) {
                     int sg = pseg[c][e];
-                    emit_window(tr, ws, b, spos[sg], slen[sg], c == 0 ? sr[sg].th : sr[sg].tl, T_O + c, true);
+                    emit_window<REC>(tr, ws, b, spos[sg], slen[sg], c == 0 ? sr[sg].th : sr[sg].tl, T_O + c, true);
                 }
             }
         }
@@ -1672,7 +1702,7 @@ __device__ void route_pair(const DevCfg& cfg, TableRef tr, WS ws, const DevBatch
             if (si[c] <= 4) {
                 for (int e = 0; e < np[c]; e++) {
                     int sg = pseg[c][e];
-                    emit_window(tr, ws, b, spos[sg], slen[sg], c == 0 ? sr[sg].th : sr[sg].tl,
+                    emit_window<REC>(tr, ws, b, spos[sg], slen[sg], c == 0 ? sr[sg].th : sr[sg].tl,
                                 (ptmp[c][e] == 0 ? T_F : T_B) + c, false);
                 }
             }
@@ -1695,16 +1725,17 @@ __device__ void route_pair(const DevCfg& cfg, TableRef tr, WS ws, const DevBatch
                 both = llo[c] == dlo && lhi[c] == dhi;
             }
             if (both) {
-                if (el) emit_window(tr, ws, b, a0, n1, ltk[c], T_O + c, true);
-                if (er) emit_window(tr, ws, b, a1, n2, rtk[c], T_O + c, true);
+                if (el) emit_window<REC>(tr, ws, b, a0, n1, ltk[c], T_O + c, true);
+                if (er) emit_window<REC>(tr, ws, b, a1, n2, rtk[c], T_O + c, true);
             }
-            if (el) emit_window(tr, ws, b, a0, n1, ltk[c], T_F + c, false);
-            if (er) emit_window(tr, ws, b, a1, n2, rtk[c], T_F + c, false);
+            if (el) emit_window<REC>(tr, ws, b, a0, n1, ltk[c], T_F + c, false);
+            if (er) emit_window<REC>(tr, ws, b, a1, n2, rtk[c], T_F + c, false);
         }
     }
 }
 
 // buffer_task_long (src/kmer.cpp:747-985)
+template <bool REC>
 __device__ void route_long(const DevCfg& cfg, TableRef tr, WS ws, const DevBatch& b, u32 u, unsigned char* scratch) {
     const int MINM = cfg.min_mer, MAXM = cfg.max_mer, SL = cfg.slice_len;
     u32 b0 = __ldg(b.bit_off + u);
@@ -1736,7 +1767,7 @@ __device__ void route_long(const DevCfg& cfg, TableRef tr, WS ws, const DevBatch
             int k[2] = {scratch[2 * (ti - 1)], scratch[2 * (ti - 1) + 1]};
 #pragma unroll
             for (int c = 0; c < 2; c++) {
-                if (!en[c] && k[c]) emit_window(tr, ws, b, b0 + s_start(ti), s_len(ti), k[c], (full[c] ? T_O : T_F) + c, full[c]);
+                if (!en[c] && k[c]) emit_window<REC>(tr, ws, b, b0 + s_start(ti), s_len(ti), k[c], (full[c] ? T_O : T_F) + c, full[c]);
                 if (!en[c] && k[c] > 0 && (ti == 1 || kk[c] == k[c])) kk[c] = k[c];
                 else en[c] = true;
             }
@@ -1749,7 +1780,7 @@ __device__ void route_long(const DevCfg& cfg, TableRef tr, WS ws, const DevBatch
             int k[2] = {sr.th, sr.tl};
 #pragma unroll
             for (int c = 0; c < 2; c++) {
-                if (!ended[c] && k[c]) emit_window(tr, ws, b, b0 + s_start(tj), s_len(tj), k[c], T_B + c, false);  // straight into 'backward'
+                if (!ended[c] && k[c]) emit_window<REC>(tr, ws, b, b0 + s_start(tj), s_len(tj), k[c], T_B + c, false);  // straight into 'backward'
                 if (sj[c] >= si[c] && !ended[c] && k[c] > 0 && (tj == snum || km[c] == k[c])) { sj[c]--; km[c] = k[c]; }
                 else ended[c] = true;
             }
@@ -1812,6 +1843,19 @@ struct StageEmit {
     }
 };
 
+// StageEmit plus one unit record per emission (the kernels' REC instantiations)
+struct RecStageEmit {
+    StageEmit add; UnitRecs* recs; u64 unit;
+    __device__ __forceinline__ void operator()(int table, int k, et::u128 key, u64 count) const {
+        add(table, k, key, count);
+        rec_append(recs, unit, table, k, (u64)key, (u64)(key >> 64), count);
+    }
+    __device__ __forceinline__ void operator()(int table, int k, et::u64 key, u64 count) const {
+        add(table, k, key, count);
+        rec_append(recs, unit, table, k, (u64)key, 0ULL, count);
+    }
+};
+
 #ifndef TREW_THREAD_BLOCK
 #define TREW_THREAD_BLOCK 128
 #endif
@@ -1843,7 +1887,8 @@ struct PlaneLoad {
     }
 };
 
-template <int MODE, class K>   // MODE 0 short single-end, 1 paired; K: u64 (MAX_MER <= 32) or u128 (<= 64)
+// MODE 0 short single-end, 1 paired; K: u64 (MAX_MER <= 32) or u128 (<= 64); REC: one unit record per emission
+template <int MODE, class K, bool REC>
 __global__ void __launch_bounds__(TREW_THREAD_BLOCK, (thread_kernel_bps<MODE, K>())) trew_exact_thread_kernel(DevCfg cfg, DevBatch b, const u32* __restrict__ survivors,
                                                                               const u32* __restrict__ n_survivors, int packed_probes,
                                                                               u32* __restrict__ hard, u32* __restrict__ n_hard,
@@ -1874,20 +1919,24 @@ __global__ void __launch_bounds__(TREW_THREAD_BLOCK, (thread_kernel_bps<MODE, K>
             entry = survivors[i];
             u32 u = entry, pm = 3u;
             if (packed_probes) { pm = entry >> kProbeShift; u &= (1u << kProbeShift) - 1u; }
-            if (MODE == 0) {
-                const u32 b0 = __ldg(b.bit_off + u);
-                const int len = (int)(__ldg(b.bit_off + u + 1) - b0);
-                if (len > et::kMaxRead) {
-                    bail = true;
-                } else {
+            auto route = [&](auto& em) {
+                if (MODE == 0) {
+                    const u32 b0 = __ldg(b.bit_off + u);
+                    const int len = (int)(__ldg(b.bit_off + u + 1) - b0);
+                    if (len > et::kMaxRead) return false;
                     PlaneLoad load{m, b.hi, b.lo, b.val, {b0, 0u}};
-                    bail = !et::route_short_thread<K>(m, len, pm & 7u, cfg.min_mer, cfg.max_mer, cfg.thr_low, cfg.thr_high, load, emit);
+                    return et::route_short_thread<K>(m, len, pm & 7u, cfg.min_mer, cfg.max_mer, cfg.thr_low, cfg.thr_high, load, em);
                 }
-            } else {
                 const u32 a0 = __ldg(b.bit_off + 2 * u), a1 = __ldg(b.bit_off + 2 * u + 1), a2 = __ldg(b.bit_off + 2 * u + 2);
                 const int n1 = (int)(a1 - a0), n2 = (int)(a2 - a1);
                 PlaneLoad load{m, b.hi, b.lo, b.val, {a0, a1}};
-                bail = !et::route_pair_thread<K>(m, n1, n2, cfg.min_mer, cfg.max_mer, cfg.thr_low, cfg.thr_high, load, emit);
+                return et::route_pair_thread<K>(m, n1, n2, cfg.min_mer, cfg.max_mer, cfg.thr_low, cfg.thr_high, load, em);
+            };
+            if constexpr (REC) {
+                RecStageEmit rem{emit, cfg.recs, cfg.unit_base + u};
+                bail = !route(rem);
+            } else {
+                bail = !route(emit);
             }
         }
         list_append(bail, entry, hard, n_hard);
@@ -1972,7 +2021,8 @@ __global__ void __launch_bounds__(256) trew_long_walk_kernel(DevCfg cfg, DevBatc
     }
 }
 
-// step 3: warp per survivor, lane per slice with emissions
+// step 3: warp per survivor, lane per slice with emissions; REC: one unit record per emission
+template <bool REC>
 __global__ void __launch_bounds__(TREW_THREAD_BLOCK, 4) trew_long_emit_kernel(DevCfg cfg, DevBatch b, LongArgs a) {
     u32* work = reinterpret_cast<u32*>(g_smem);
     u64* s_key = reinterpret_cast<u64*>(work + et::Lay<et::u64>::WORDS * TREW_THREAD_BLOCK);
@@ -2004,7 +2054,12 @@ __global__ void __launch_bounds__(TREW_THREAD_BLOCK, 4) trew_long_emit_kernel(De
                 const bool folded = (byte & 0x80u) != 0u;
                 const int table = (f >= 2 ? et::T_B : (folded ? et::T_O : et::T_F)) + c;
                 et::LongTask tk{(unsigned short)t, (unsigned char)(byte & 0x7fu), (unsigned char)(table | (folded ? 8 : 0))};
-                et::long_emit(m, g, tk, load, x, emit);
+                if constexpr (REC) {
+                    RecStageEmit rem{emit, cfg.recs, cfg.unit_base + u};
+                    et::long_emit(m, g, tk, load, x, rem);
+                } else {
+                    et::long_emit(m, g, tk, load, x, emit);
+                }
             }
         }
     }
@@ -2034,7 +2089,8 @@ void launch_long_thread(const DevCfg& cfg, const DevBatch& b, const unsigned int
     const size_t smem_stats = (size_t)et::Lay<et::u64>::WORDS * TREW_THREAD_BLOCK * sizeof(u32);
     trew_long_stats_kernel<<<sm_count * 4, TREW_THREAD_BLOCK, smem_stats, stream>>>(cfg, b, a);
     trew_long_walk_kernel<<<sm_count * 2, 256, 0, stream>>>(cfg, b, a);
-    trew_long_emit_kernel<<<sm_count * 4, TREW_THREAD_BLOCK, kThreadKernelSmem, stream>>>(cfg, b, a);
+    if (cfg.recs) trew_long_emit_kernel<true><<<sm_count * 4, TREW_THREAD_BLOCK, kThreadKernelSmem, stream>>>(cfg, b, a);
+    else trew_long_emit_kernel<false><<<sm_count * 4, TREW_THREAD_BLOCK, kThreadKernelSmem, stream>>>(cfg, b, a);
 }
 
 // true when the thread kernel can take (most of) a batch: short single-end or paired mode, 64-bit units
@@ -2049,16 +2105,20 @@ void launch_exact_thread(const DevCfg& cfg, const DevBatch& b, const unsigned in
                          int blocks_per_sm, unsigned int* work_counter, cudaStream_t stream) {
     const bool wide = cfg.max_mer > 32;
     // blocks_per_sm 0: as many as the kernel was built to have resident (one wave)
-#define TREW_LAUNCH_THREAD(MODE, K)                                                                                               \
-    trew_exact_thread_kernel<MODE, K><<<sm_count * (blocks_per_sm > 0 ? blocks_per_sm : thread_kernel_bps<MODE, K>()),            \
-                                        TREW_THREAD_BLOCK, thread_kernel_smem<K>(), stream>>>(                                    \
+#define TREW_LAUNCH_THREAD(MODE, K, REC)                                                                                          \
+    trew_exact_thread_kernel<MODE, K, REC><<<sm_count * (blocks_per_sm > 0 ? blocks_per_sm : thread_kernel_bps<MODE, K>()),       \
+                                             TREW_THREAD_BLOCK, thread_kernel_smem<K>(), stream>>>(                               \
         cfg, b, survivors, n_survivors, packed_probes, hard, n_hard, total_survivors, work_counter)
-    if (cfg.mode == 0) { if (wide) TREW_LAUNCH_THREAD(0, et::u128); else TREW_LAUNCH_THREAD(0, et::u64); }
-    else               { if (wide) TREW_LAUNCH_THREAD(1, et::u128); else TREW_LAUNCH_THREAD(1, et::u64); }
+#define TREW_LAUNCH_THREAD_MODE(MODE)                                                                                             \
+    if (cfg.recs) { if (wide) TREW_LAUNCH_THREAD(MODE, et::u128, true); else TREW_LAUNCH_THREAD(MODE, et::u64, true); }            \
+    else          { if (wide) TREW_LAUNCH_THREAD(MODE, et::u128, false); else TREW_LAUNCH_THREAD(MODE, et::u64, false); }
+    if (cfg.mode == 0) { TREW_LAUNCH_THREAD_MODE(0) }
+    else               { TREW_LAUNCH_THREAD_MODE(1) }
+#undef TREW_LAUNCH_THREAD_MODE
 #undef TREW_LAUNCH_THREAD
 }
 
-template <int MODE>
+template <int MODE, bool REC>   // REC: one unit record per class added
 __global__ void __launch_bounds__(kExactWarps * 32, TREW_EXACT_BPS) trew_exact_kernel(DevCfg cfg, DevBatch b, ExactArgs a) {
     const int wid = threadIdx.x >> 5;
     const u32 lane = lane_id();
@@ -2067,6 +2127,10 @@ __global__ void __launch_bounds__(kExactWarps * 32, TREW_EXACT_BPS) trew_exact_k
     ws.off = (u32)((size_t)wid * exact_warp_bytes(a.run_cap)); ws.lane = lane; ws.flags = a.exp_flags;
     TableRef tr{cfg.slots, cfg.slot_mask, cfg.error_flag};
     ws.hdr()[lane] = lane == HD_CUR_LEN || lane == HD_EV_LEN || lane == HD_EV_K ? 0xffffffffu : 0u;
+    if constexpr (REC) {
+        if (lane == HD_UNIT_BASE) { ws.hdr()[lane] = (u32)cfg.unit_base; ws.hdr()[lane + 1] = (u32)(cfg.unit_base >> 32); }
+        if (lane == HD_RECS) { ws.hdr()[lane] = (u32)(u64)cfg.recs; ws.hdr()[lane + 1] = (u32)((u64)cfg.recs >> 32); }
+    }
     __syncwarp();
     const u32 n = *a.n_survivors;
     if (blockIdx.x == 0 && threadIdx.x == 0 && a.total_survivors) atomicAdd(a.total_survivors, (u64)n);
@@ -2078,9 +2142,10 @@ __global__ void __launch_bounds__(kExactWarps * 32, TREW_EXACT_BPS) trew_exact_k
         if (idx >= n) break;
         u32 u = a.reverse ? *(a.survivors - idx) : a.survivors[idx], pm = 0xfu;
         if (a.packed_probes) { pm = u >> kProbeShift; u &= (1u << kProbeShift) - 1u; }
-        if constexpr (MODE == 0) route_short(cfg, tr, ws, b, u, pm);
-        else if constexpr (MODE == 1) route_pair(cfg, tr, ws, b, u);
-        else route_long(cfg, tr, ws, b, u, scratch);
+        if constexpr (REC) ws.hdr()[HD_UNIT] = u;   // for emit_classes (every lane stores the same value)
+        if constexpr (MODE == 0) route_short<REC>(cfg, tr, ws, b, u, pm);
+        else if constexpr (MODE == 1) route_pair<REC>(cfg, tr, ws, b, u);
+        else route_long<REC>(cfg, tr, ws, b, u, scratch);
     }
 }
 
@@ -2089,15 +2154,26 @@ int exact_warps_total(int sm_count) { return sm_count * kExactBlocksPerSM * kExa
 
 cudaError_t prepare_exact(int run_cap_max) {
     int bytes = (int)exact_smem_bytes(run_cap_max, true);
-    cudaError_t e = cudaFuncSetAttribute(trew_exact_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(trew_exact_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(trew_exact_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(trew_exact_thread_kernel<0, et::u64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)thread_kernel_smem<et::u64>());
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(trew_exact_thread_kernel<1, et::u64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)thread_kernel_smem<et::u64>());
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(trew_exact_thread_kernel<0, et::u128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)thread_kernel_smem<et::u128>());
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(trew_exact_thread_kernel<1, et::u128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)thread_kernel_smem<et::u128>());
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(trew_long_stats_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kThreadKernelSmem);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(trew_long_emit_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kThreadKernelSmem);
+    cudaError_t e = cudaSuccess;
+#define TREW_SMEM_ATTR(F, BYTES) if (e == cudaSuccess) e = cudaFuncSetAttribute(F, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(BYTES))
+    TREW_SMEM_ATTR((trew_exact_kernel<0, false>), bytes);
+    TREW_SMEM_ATTR((trew_exact_kernel<1, false>), bytes);
+    TREW_SMEM_ATTR((trew_exact_kernel<2, false>), bytes);
+    TREW_SMEM_ATTR((trew_exact_kernel<0, true>), bytes);
+    TREW_SMEM_ATTR((trew_exact_kernel<1, true>), bytes);
+    TREW_SMEM_ATTR((trew_exact_kernel<2, true>), bytes);
+    TREW_SMEM_ATTR((trew_exact_thread_kernel<0, et::u64, false>), thread_kernel_smem<et::u64>());
+    TREW_SMEM_ATTR((trew_exact_thread_kernel<1, et::u64, false>), thread_kernel_smem<et::u64>());
+    TREW_SMEM_ATTR((trew_exact_thread_kernel<0, et::u128, false>), thread_kernel_smem<et::u128>());
+    TREW_SMEM_ATTR((trew_exact_thread_kernel<1, et::u128, false>), thread_kernel_smem<et::u128>());
+    TREW_SMEM_ATTR((trew_exact_thread_kernel<0, et::u64, true>), thread_kernel_smem<et::u64>());
+    TREW_SMEM_ATTR((trew_exact_thread_kernel<1, et::u64, true>), thread_kernel_smem<et::u64>());
+    TREW_SMEM_ATTR((trew_exact_thread_kernel<0, et::u128, true>), thread_kernel_smem<et::u128>());
+    TREW_SMEM_ATTR((trew_exact_thread_kernel<1, et::u128, true>), thread_kernel_smem<et::u128>());
+    TREW_SMEM_ATTR(trew_long_stats_kernel, kThreadKernelSmem);
+    TREW_SMEM_ATTR(trew_long_emit_kernel<false>, kThreadKernelSmem);
+    TREW_SMEM_ATTR(trew_long_emit_kernel<true>, kThreadKernelSmem);
+#undef TREW_SMEM_ATTR
     return e;
 }
 
@@ -2110,9 +2186,15 @@ LaunchPlan default_launch_plan(int sm_count) { return LaunchPlan{sm_count * 128,
 void launch_exact(const DevCfg& cfg, const DevBatch& b, const ExactArgs& a, const LaunchPlan& plan, cudaStream_t stream) {
     size_t smem = exact_smem_bytes(a.run_cap, true);
     dim3 grid(plan.exact_blocks), block(kExactWarps * 32);
-    if (cfg.mode == 0) trew_exact_kernel<0><<<grid, block, smem, stream>>>(cfg, b, a);
-    else if (cfg.mode == 1) trew_exact_kernel<1><<<grid, block, smem, stream>>>(cfg, b, a);
-    else trew_exact_kernel<2><<<grid, block, smem, stream>>>(cfg, b, a);
+    if (cfg.recs) {
+        if (cfg.mode == 0) trew_exact_kernel<0, true><<<grid, block, smem, stream>>>(cfg, b, a);
+        else if (cfg.mode == 1) trew_exact_kernel<1, true><<<grid, block, smem, stream>>>(cfg, b, a);
+        else trew_exact_kernel<2, true><<<grid, block, smem, stream>>>(cfg, b, a);
+    } else {
+        if (cfg.mode == 0) trew_exact_kernel<0, false><<<grid, block, smem, stream>>>(cfg, b, a);
+        else if (cfg.mode == 1) trew_exact_kernel<1, false><<<grid, block, smem, stream>>>(cfg, b, a);
+        else trew_exact_kernel<2, false><<<grid, block, smem, stream>>>(cfg, b, a);
+    }
 }
 
 }  // namespace trew

@@ -33,6 +33,13 @@ struct __align__(32) Slot {
     unsigned int state;  // 0 empty, 1 being written, 2 ready
 };
 
+// per-unit hit records (device memory): rows are appended at n, which keeps counting past cap
+struct UnitRecs {
+    trew_unit_record* buf;
+    unsigned long long cap;
+    unsigned long long n;
+};
+
 struct DevCfg {
     int mode, min_mer, max_mer, slice_len;
     double low, high;
@@ -41,6 +48,8 @@ struct DevCfg {
     unsigned int* error_flag;        // [0] set to TREW_ERR_TABLE_FULL on overflow, [1] number of distinct keys inserted
     const unsigned short* thr_low;   // kThrTableSize entries: min M with (double)M/(double)T >= low; 0xFFFF for T = 0
     const unsigned short* thr_high;  // the same for the high baseline
+    UnitRecs* recs;                  // nullptr: no records
+    unsigned long long unit_base;    // ordinal of the batch's unit 0
 };
 
 struct DevBatch {
@@ -108,6 +117,11 @@ cudaError_t filter_report_rows(const trew_entry* d_rows, unsigned int n, unsigne
 // validity plane from n 12-byte records (u32 block position, u64 mask of invalid bases): clears those bits of val
 void launch_clear_invalid(unsigned int* val, const unsigned int* rec, unsigned int n, cudaStream_t stream);
 void launch_merge_entries(const DevCfg& cfg, const trew_entry* entries, unsigned int n, cudaStream_t stream);
+
+// unit records -> sorted by (unit, table, k, seq_hi, seq_lo) into d_out, equal keys summed, *d_n_out rows; wide = some key
+// uses seq_hi; d_temp == nullptr queries *temp_bytes
+cudaError_t sort_combine_records(const trew_unit_record* d_in, unsigned int n, bool wide, trew_unit_record* d_out, unsigned int* d_n_out,
+                                 void* d_temp, size_t* temp_bytes, cudaStream_t stream);
 
 // flavor 0: single reads (configs[1]); 1: pairs -- reads 2u, 2u+1 are the two ends of one fragment, both telomeric or
 // neither, mate 2 on the opposite strand (configs[2]); 2: long reads whose first or last 0.5-5 kb are telomeric (configs[3])

@@ -186,6 +186,101 @@ cudaError_t combine_sorted_rows(const trew_entry* d_sorted, unsigned int n, trew
     return cudaGetLastError();
 }
 
+// ---- unit records: sort by (unit, table, k, seq_hi, seq_lo) the way sort_entries_radix sorts rows -- stable LSD passes over
+// the key fields with a row index as payload, one gather -- then sum the rows of equal keys as combine_sorted_rows does.
+
+__global__ void key_from_records_kernel(const trew_unit_record* __restrict__ r, const u32* __restrict__ idx, u32 n, int which,
+                                        u64* __restrict__ key64, unsigned short* __restrict__ key16, u32* __restrict__ idx_out) {
+    for (u32 i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        const u32 j = idx ? idx[i] : i;
+        if (which == 0) { key64[i] = r[j].seq_lo; idx_out[i] = i; }
+        else if (which == 1) key64[i] = r[j].seq_hi;
+        else if (which == 2) key16[i] = (unsigned short)(((u32)r[j].table << 8) | (u32)r[j].k);
+        else key64[i] = r[j].unit;
+    }
+}
+
+__device__ __forceinline__ bool same_record_key(const trew_unit_record& a, const trew_unit_record& b) {
+    return a.unit == b.unit && a.seq_lo == b.seq_lo && a.seq_hi == b.seq_hi && a.table == b.table && a.k == b.k;
+}
+
+// gathers the sorted order and flags the first row of every key
+__global__ void gather_records_kernel(const trew_unit_record* __restrict__ r, const u32* __restrict__ idx, u32 n,
+                                      trew_unit_record* __restrict__ out, u32* __restrict__ flags) {
+    for (u32 i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        out[i] = r[idx[i]];
+        flags[i] = (i == 0 || !same_record_key(r[idx[i]], r[idx[i - 1]])) ? 1u : 0u;
+    }
+}
+
+__global__ void combine_records_kernel(const trew_unit_record* __restrict__ r, u32 n, const u32* __restrict__ flags,
+                                       const u32* __restrict__ pos, trew_unit_record* __restrict__ out, u32* __restrict__ n_out) {
+    for (u32 i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        if (!flags[i]) continue;
+        trew_unit_record x = r[i];
+        for (u32 j = i + 1; j < n && !flags[j]; j++) x.count += r[j].count;
+        out[pos[i]] = x;
+    }
+    if (blockIdx.x == 0 && threadIdx.x == 0) *n_out = n ? pos[n - 1] + flags[n - 1] : 0u;
+}
+
+cudaError_t sort_combine_records(const trew_unit_record* d_in, unsigned int n, bool wide, trew_unit_record* d_out, unsigned int* d_n_out,
+                                 void* d_temp, size_t* temp_bytes, cudaStream_t stream) {
+    size_t cub64 = 0, cub16 = 0, scan_bytes = 0;
+    cub::DoubleBuffer<u64> k64(nullptr, nullptr);
+    cub::DoubleBuffer<unsigned short> k16(nullptr, nullptr);
+    cub::DoubleBuffer<u32> ix(nullptr, nullptr);
+    cudaError_t e = cub::DeviceRadixSort::SortPairs(nullptr, cub64, k64, ix, (int)n, 0, 64, stream);
+    if (e != cudaSuccess) return e;
+    e = cub::DeviceRadixSort::SortPairs(nullptr, cub16, k16, ix, (int)n, 0, 11, stream);
+    if (e != cudaSuccess) return e;
+    e = cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, (u32*)nullptr, (u32*)nullptr, (int)n, stream);
+    if (e != cudaSuccess) return e;
+    const size_t cub_bytes = align256(std::max(std::max(cub64, cub16), scan_bytes));
+    const size_t rows = align256((size_t)n * sizeof(trew_unit_record));
+    const size_t need = 2 * align256((size_t)n * 8) + 4 * align256((size_t)n * 4) + 2 * align256((size_t)n * 2) + rows + cub_bytes;
+    if (!d_temp) { *temp_bytes = need; return cudaSuccess; }
+    if (*temp_bytes < need) return cudaErrorInvalidValue;
+    char* p = (char*)d_temp;
+    u64* ka = (u64*)p; p += align256((size_t)n * 8);
+    u64* kb = (u64*)p; p += align256((size_t)n * 8);
+    u32* ia = (u32*)p; p += align256((size_t)n * 4);
+    u32* ib = (u32*)p; p += align256((size_t)n * 4);
+    u32* flags = (u32*)p; p += align256((size_t)n * 4);
+    u32* pos = (u32*)p; p += align256((size_t)n * 4);
+    unsigned short* sa = (unsigned short*)p; p += align256((size_t)n * 2);
+    unsigned short* sb = (unsigned short*)p; p += align256((size_t)n * 2);
+    trew_unit_record* sorted = (trew_unit_record*)p; p += rows;
+    void* cub_tmp = p;
+    const int blocks = (int)std::min<unsigned int>((n + 255) / 256, 4736u);
+    if (n) {
+        k64 = cub::DoubleBuffer<u64>(ka, kb);
+        ix = cub::DoubleBuffer<u32>(ia, ib);
+        k16 = cub::DoubleBuffer<unsigned short>(sa, sb);
+        size_t tb;
+        key_from_records_kernel<<<blocks, 256, 0, stream>>>(d_in, nullptr, n, 0, k64.Current(), nullptr, ix.Current());
+        e = cub::DeviceRadixSort::SortPairs(cub_tmp, tb = cub_bytes, k64, ix, (int)n, 0, 64, stream);
+        if (e != cudaSuccess) return e;
+        if (wide) {
+            key_from_records_kernel<<<blocks, 256, 0, stream>>>(d_in, ix.Current(), n, 1, k64.Current(), nullptr, nullptr);
+            e = cub::DeviceRadixSort::SortPairs(cub_tmp, tb = cub_bytes, k64, ix, (int)n, 0, 64, stream);
+            if (e != cudaSuccess) return e;
+        }
+        key_from_records_kernel<<<blocks, 256, 0, stream>>>(d_in, ix.Current(), n, 2, nullptr, k16.Current(), nullptr);
+        e = cub::DeviceRadixSort::SortPairs(cub_tmp, tb = cub_bytes, k16, ix, (int)n, 0, 11, stream);
+        if (e != cudaSuccess) return e;
+        key_from_records_kernel<<<blocks, 256, 0, stream>>>(d_in, ix.Current(), n, 3, k64.Current(), nullptr, nullptr);
+        e = cub::DeviceRadixSort::SortPairs(cub_tmp, tb = cub_bytes, k64, ix, (int)n, 0, 64, stream);
+        if (e != cudaSuccess) return e;
+        gather_records_kernel<<<blocks, 256, 0, stream>>>(d_in, ix.Current(), n, sorted, flags);
+    }
+    size_t sb2 = cub_bytes;
+    e = cub::DeviceScan::ExclusiveSum(cub_tmp, sb2, flags, pos, (int)n, stream);
+    if (e != cudaSuccess) return e;
+    combine_records_kernel<<<n ? blocks : 1, 256, 0, stream>>>(sorted, n, flags, pos, d_out, d_n_out);
+    return cudaGetLastError();
+}
+
 // ---- report filter: only the rows that can reach the report of a one-file run ------------------------------------------
 //
 // process_output prints an entry when forward + backward + both >= 10 (ABS_MIN_PRINT_COUNT, src/kmer.cpp:1615-1620) and

@@ -21,12 +21,13 @@ const char* kVersion = "0.5.0";
 void usage(const std::string& cmd) {
     if (cmd == "long") {
         std::cerr << "Usage: long [--help] [--version] [--thread THREAD] [--table_max_mer TABLE_MAX_MER] [--low_baseline LOW_BASELINE] "
-                     "[--high_baseline HIGH_BASELINE] [--slice_length SLICE_LENGTH] [--queue_size QUEUE_SIZE] MIN_MER MAX_MER LONG_FASTQ...\n\n"
+                     "[--high_baseline HIGH_BASELINE] [--slice_length SLICE_LENGTH] [--queue_size QUEUE_SIZE] [--read_hits READ_HITS] "
+                     "MIN_MER MAX_MER LONG_FASTQ...\n\n"
                      "Estimate TRM from long-read sequencing data.\n";
     } else if (cmd == "short") {
         std::cerr << "Usage: short [--help] [--version] [--thread THREAD] [--paired_end] [--fq1 FASTQ_FRONT...] [--fq2 FASTQ_REVERSE...] "
                      "[--table_max_mer TABLE_MAX_MER] [--low_baseline LOW_BASELINE] [--high_baseline HIGH_BASELINE] "
-                     "[--queue_size QUEUE_SIZE] MIN_MER MAX_MER SHORT_FASTQ...\n\n"
+                     "[--queue_size QUEUE_SIZE] [--read_hits READ_HITS] MIN_MER MAX_MER SHORT_FASTQ...\n\n"
                      "Estimate TRM from short-read sequencing data.\n";
     } else {
         std::cerr << "Usage: trew [--help] [--version] {long,short}\n\nSubcommands:\n"
@@ -56,6 +57,24 @@ bool has_gz_ext(const std::filesystem::path& p) {  // src/trew.cpp:407, 422-433
     return e == ".gz" || e == ".bgz";
 }
 
+// --read_hits: one TSV line per unit record of a file -- file, record (0-based FASTQ record / pair index), table, k, the repeat
+// unit as bases (the reference's 2-bit code T=0 G=1 C=2 A=3, first base in the most significant bits) and the count
+void write_read_hits(FILE* out, const std::string& file, const trew_unit_record* r, uint64_t n) {
+    static const char* kTable[6] = {"F_h", "F_l", "B_h", "B_l", "O_h", "O_l"};
+    std::string unit;
+    for (uint64_t i = 0; i < n; i++) {
+        const int k = r[i].k;
+        unit.resize((size_t)k);
+        for (int j = 0; j < k; j++) {
+            const int sh = 2 * (k - 1 - j);
+            const uint64_t code = sh >= 64 ? (r[i].seq_hi >> (sh - 64)) & 3u : (r[i].seq_lo >> sh) & 3u;
+            unit[(size_t)j] = "TGCA"[code];
+        }
+        fprintf(out, "%s\t%llu\t%s\t%d\t%s\t%u\n", file.c_str(), (unsigned long long)r[i].unit, kTable[r[i].table % 6], k, unit.c_str(),
+                r[i].count);
+    }
+}
+
 }  // namespace
 
 int main(int argc, char** argv) {
@@ -69,6 +88,7 @@ int main(int argc, char** argv) {
     int min_mer = 0, max_mer = 0, num_thread = 2, table_max_mer = 12, slice_length = 150, queue_size = -1;
     double low = 0.5, high = 0.8;
     bool paired = false, used_fq1 = false, used_fq2 = false;
+    const char* read_hits = nullptr;
     std::vector<std::string> positional, fq1, fq2;
     std::vector<std::string>* sink = &positional;
     // argparse also takes `--name=value` and a value glued to a short option (`-t4`): split those first
@@ -96,6 +116,7 @@ int main(int argc, char** argv) {
         else if (!is_short && (a == "-s" || a == "--slice_length")) { ok = value(&v) && parse_int(v, &slice_length); sink = &positional; }
         else if (a == "-q" || a == "--queue_size") { ok = value(&v) && parse_int(v, &queue_size); sink = &positional; }
         else if (is_short && a == "--paired_end") { paired = true; sink = &positional; }
+        else if (a == "--read_hits") { ok = value(&read_hits); sink = &positional; }
         else if (is_short && a == "--fq1") { used_fq1 = true; sink = &fq1; }
         else if (is_short && a == "--fq2") { used_fq2 = true; sink = &fq2; }
         else if (a.size() > 1 && a[0] == '-' && !(a[1] >= '0' && a[1] <= '9')) ok = false;
@@ -199,6 +220,17 @@ int main(int argc, char** argv) {
     if (timing) fprintf(stderr, "[trew] contexts on %d device(s): %.1f ms\n", trew_multi_device_count(ctx), now() - t_start);
     trew_report* rep = nullptr;
     trew_report_create(min_mer, &rep);
+    // --read_hits: unit records, sized from the input (a file that needs more is scanned again with what it needed)
+    FILE* hits = nullptr;
+    uint64_t rec_cap = 0;
+    if (read_hits) {
+        hits = fopen(read_hits, "w");
+        if (!hits) { fprintf(stderr, "%s : cannot open for writing\n", read_hits); trew_report_destroy(rep); trew_multi_destroy(ctx); return 1; }
+        uintmax_t input_bytes = 0;
+        for (auto& p : paths) { std::error_code ec; uintmax_t sz = std::filesystem::file_size(p, ec); if (!ec) input_bytes += has_gz_ext(p) ? 4 * sz : sz; }
+        rec_cap = std::min<uint64_t>(std::max<uint64_t>(input_bytes / 128, 1u << 12), 1u << 26);   // 2.4 per 150-base FASTQ record
+        trew_multi_enable_unit_records(ctx, rec_cap);
+    }
 
     const bool is_pair = cfg.mode == TREW_MODE_PAIR;
     size_t printed = 0;   // bytes of the report text already written to stdout
@@ -227,6 +259,30 @@ int main(int argc, char** argv) {
             return 1;
         }
         trew_report_add_file(rep, a.c_str(), entries, n);
+        if (hits) {
+            const trew_unit_record* recs = nullptr;
+            uint64_t nr = 0;
+            rc = trew_multi_unit_records(ctx, &recs, &nr);
+            unsigned long long need = 0;
+            const char* why = trew_multi_last_error(ctx);
+            const char* at = rc == TREW_ERR_TABLE_FULL && why ? strstr(why, "a capacity of ") : nullptr;
+            if (at && sscanf(at, "a capacity of %llu", &need) == 1) {   // once more, with the capacity that is enough
+                rec_cap = need;
+                rc = trew_multi_reset(ctx);
+                if (rc == TREW_OK) rc = trew_multi_enable_unit_records(ctx, rec_cap);
+                if (rc == TREW_OK) rc = trew_multi_process_file(ctx, a.c_str(), g1, is_pair ? b.c_str() : nullptr, g2);
+                if (rc == TREW_OK) rc = trew_multi_unit_records(ctx, &recs, &nr);
+            }
+            if (rc != TREW_OK) {
+                fprintf(stderr, "%s\n", trew_multi_last_error(ctx));
+                fclose(hits);
+                trew_report_destroy(rep);
+                trew_multi_destroy(ctx);
+                return 1;
+            }
+            write_read_hits(hits, a, recs, nr);
+            fflush(hits);
+        }
         // each file's sections go out as soon as they are ready, like process_output prints them (src/kmer.cpp:1615-1631):
         // a later file that fails leaves the earlier sections on stdout
         const char* part = nullptr;
@@ -241,6 +297,7 @@ int main(int argc, char** argv) {
     trew_report_finish(rep, &text, &len);
     fwrite(text + printed, 1, len - printed, stdout);
     trew_report_destroy(rep);
+    if (hits) fclose(hits);
     const double t_done = now();
     trew_multi_destroy(ctx);
     if (timing) fprintf(stderr, "[trew] report %.1f ms after the last file, teardown %.1f ms, total %.1f ms\n", t_done - t_start, now() - t_done, now() - t_start);
