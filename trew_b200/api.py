@@ -69,7 +69,7 @@ ABI_SYMBOLS = [
     "trew_multi_device_count", "trew_multi_last_error", "trew_multi_submit_chunk", "trew_multi_process_file",
     "trew_multi_reset", "trew_multi_finish", "trew_multi_get_stats", "trew_multi_ctx", "trew_dev_set_report_filter",
     "trew_multi_set_report_filter", "trew_dev_enable_unit_records", "trew_dev_unit_records", "trew_multi_enable_unit_records",
-    "trew_multi_unit_records",
+    "trew_multi_unit_records", "trew_check_batch",
 ]
 
 # trew_unit_record: one unit's adds to one (table, k, seq), sorted by (unit, table, k, seq_hi, seq_lo)
@@ -114,6 +114,7 @@ def load_library() -> C.CDLL:
     L.trew_dev_submit_chunk.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint32]
     L.trew_dev_submit_packed.argtypes = [C.c_void_p, C.POINTER(Batch)]
     L.trew_dev_upload.argtypes = [C.c_void_p, C.POINTER(Batch), C.POINTER(C.c_void_p)]
+    L.trew_check_batch.argtypes = [C.c_int, C.POINTER(Batch)]
     L.trew_dev_scan_resident.argtypes = [C.c_void_p, C.c_void_p]
     L.trew_dev_free_resident.argtypes = [C.c_void_p, C.c_void_p]
     L.trew_dev_free_resident.restype = None
@@ -310,6 +311,9 @@ class DeviceContext:
             self.submit_chunk(b1, l1)
 
     def submit_packed(self, pb: PackedBatch, max_read_len: Optional[int] = None) -> None:
+        """max_read_len, when given, replaces the packer's value in pb.batch (at least the longest read, or TREW_ERR_ARG)."""
+        if max_read_len is not None:
+            pb.batch.max_read_len = max_read_len
         self._check(self.lib.trew_dev_submit_packed(self.ctx, C.byref(pb.batch)))
 
     def upload(self, pb: PackedBatch) -> C.c_void_p:

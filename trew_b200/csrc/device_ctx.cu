@@ -500,6 +500,30 @@ int fork_aux(trew_ctx* ctx) {
 // are the same.
 int reader_slice_length(const trew_ctx* ctx) { return ctx->d_recs ? 0 : ctx->cfg.slice_length; }
 
+// A packed batch as the caller describes it, checked against what the scan relies on: offsets that start at 0 and never
+// decrease, whole pairs, submit_chunk's length limits, and a max_read_len no smaller than the longest read (it sizes the
+// exact kernel's run capacity, the long-read scratch stride and the filter variant).  One pass over bit_off.
+int check_batch(trew_ctx* ctx, int mode, const trew_batch* batch) {
+    if (!batch) return fail(ctx, TREW_ERR_ARG, "null batch");
+    const uint32_t n = batch->n_reads;
+    if (n == 0) return TREW_OK;
+    if (!batch->bit_off) return fail(ctx, TREW_ERR_ARG, "null bit_off");
+    if (batch->bit_off[0] != 0) return fail(ctx, TREW_ERR_ARG, "bit_off[0] must be 0");
+    if (mode == TREW_MODE_PAIR && (n & 1u)) return fail(ctx, TREW_ERR_ARG, "paired batch with an odd n_reads (%u): mates come in twos", n);
+    uint32_t longest = 0;
+    for (uint32_t i = 0; i < n; i++) {
+        const uint32_t a = batch->bit_off[i], b = batch->bit_off[i + 1];
+        if (b < a) return fail(ctx, TREW_ERR_ARG, "bit_off decreases at read %u (%u after %u)", i, b, a);
+        longest = std::max(longest, b - a);
+    }
+    if (mode == TREW_MODE_SHORT && longest > 1000)  // MAX_SEQ, src/kmer.cpp:1006-1008
+        return fail(ctx, TREW_ERR_TOO_LONG, "%s", trew_status_string(TREW_ERR_TOO_LONG));
+    if (mode == TREW_MODE_PAIR && longest > (uint32_t)kMaxWindow) return fail(ctx, TREW_ERR_TOO_LONG, "paired read longer than %d", kMaxWindow);
+    if (batch->max_read_len < longest)
+        return fail(ctx, TREW_ERR_ARG, "max_read_len (%u) is smaller than the longest read (%u)", batch->max_read_len, longest);
+    return TREW_OK;
+}
+
 int check_device_error(trew_ctx* ctx) {
     unsigned int e = 0;
     CK(cudaMemcpy(&e, ctx->d_error, sizeof(e), cudaMemcpyDeviceToHost));
@@ -526,6 +550,11 @@ const char* trew_status_string(int status) {
         case TREW_ERR_NOMEM: return "memory allocation failure";
         default: return "unknown status";
     }
+}
+
+int trew_check_batch(int mode, const trew_batch* batch) {
+    if (mode < TREW_MODE_SHORT || mode > TREW_MODE_LONG) return TREW_ERR_ARG;
+    return check_batch(nullptr, mode, batch);
 }
 
 // trew_dev_create has no context to hang its message on: it is kept here and read with trew_dev_last_error(NULL)
@@ -723,6 +752,8 @@ int trew_dev_submit_chunk(trew_ctx* ctx, const char* buffer1, const int32_t* loc
 
 int trew_dev_submit_packed(trew_ctx* ctx, const trew_batch* batch) {
     if (!ctx || !batch) return TREW_ERR_ARG;
+    int rc = check_batch(ctx, ctx->cfg.mode, batch);
+    if (rc) return rc;
     CK(cudaSetDevice(ctx->cfg.device));
     uint32_t n = batch->n_reads;
     if (n == 0) return TREW_OK;
@@ -730,10 +761,9 @@ int trew_dev_submit_packed(trew_ctx* ctx, const trew_batch* batch) {
     size_t bytes = batch_bytes(n, bases);
     if (bytes > ctx->staging_bytes || n > ctx->slots[0].survivors_cap)
         return fail(ctx, TREW_ERR_ARG, "packed batch (%zu bytes) larger than a staging buffer (%zu)", bytes, ctx->staging_bytes);
-    if (batch->bit_off[0] != 0) return fail(ctx, TREW_ERR_ARG, "bit_off[0] must be 0");
     SlotRes& s = ctx->slots[ctx->next_slot];
     ctx->next_slot = (ctx->next_slot + 1) % ctx->slots.size();
-    int rc = retire_slot(ctx, s);
+    rc = retire_slot(ctx, s);
     if (rc) return rc;
     BatchView v;
     batch_layout(s.h_buf, n, bases, &v);
@@ -764,6 +794,8 @@ int trew_dev_submit_packed(trew_ctx* ctx, const trew_batch* batch) {
 
 int trew_dev_upload(trew_ctx* ctx, const trew_batch* batch, trew_resident** out) {
     if (!ctx || !batch || !out) return TREW_ERR_ARG;
+    int rc = check_batch(ctx, ctx->cfg.mode, batch);
+    if (rc) return rc;
     CK(cudaSetDevice(ctx->cfg.device));
     uint32_t n = batch->n_reads;
     uint64_t bases = n ? batch->bit_off[n] : 0;
