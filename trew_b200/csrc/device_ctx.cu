@@ -1025,7 +1025,8 @@ int trew_dev_finish_merged(trew_ctx* ctx, const trew_entry* const* d_lists, cons
     if (rc) return rc;
     uint64_t total = n0;
     for (uint32_t i = 0; i < n_lists; i++) total += n_rows[i];
-    if (total > 0xfffffff0ULL) return fail(ctx, TREW_ERR_ARG, "too many rows to merge (%llu)", (unsigned long long)total);
+    // the sort and the scans below count rows in an int
+    if (total > 0x7fffffffULL) return fail(ctx, TREW_ERR_ARG, "too many rows to merge (%llu)", (unsigned long long)total);
     // concatenate, sort, sum the counts of equal keys: the union of the tables without touching this context's table
     CK(ctx->d_concat.grow((size_t)total, ctx->main_stream));
     uint64_t at = 0;

@@ -317,14 +317,16 @@ __device__ __forceinline__ u64 filt_tag(const trew_entry& e) {
     return x | 1ULL;   // 0 = empty slot
 }
 
-struct FiltGroup { u64 tag; u32 tot[2]; };
+// 64-bit totals: the clamped adds (each at most min_total < 2^32) of up to 2^32 rows cannot wrap them, so a group far above
+// min_total is never dropped because its sum passed 2^32
+struct FiltGroup { u64 tag; u64 tot[2]; };
 
 __global__ void filter_accumulate_kernel(const trew_entry* __restrict__ e, u32 n, FiltGroup* __restrict__ g, u32 gmask, u32 cap_add,
                                          u64* __restrict__ tags) {
     for (u32 i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
         const u64 tag = filt_tag(e[i]);
         tags[i] = tag;
-        const u32 add = (u32)(e[i].count < (u64)cap_add ? e[i].count : (u64)cap_add);   // saturating: only ">= min_total" matters
+        const u64 add = e[i].count < (u64)cap_add ? e[i].count : (u64)cap_add;   // saturating: only ">= min_total" matters
         u32 s = (u32)(tag >> 20) & gmask;
         for (;;) {
             const u64 old = atomicCAS((unsigned long long*)&g[s].tag, 0ULL, (unsigned long long)tag);
@@ -340,7 +342,7 @@ __global__ void filter_flags_kernel(const trew_entry* __restrict__ e, u32 n, con
         const u64 tag = tags[i];
         u32 s = (u32)(tag >> 20) & gmask;
         while (g[s].tag != tag) s = (s + 1) & gmask;
-        flags[i] = (g[s].tot[0] >= min_total || g[s].tot[1] >= min_total) ? 1u : 0u;
+        flags[i] = (g[s].tot[0] >= (u64)min_total || g[s].tot[1] >= (u64)min_total) ? 1u : 0u;
     }
 }
 
